@@ -3,7 +3,7 @@
 samples, 8x256 MLP; % of tensor-core roofline).
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c2|c3|c4|c5]
-                  [--scaling weak|strong] [--precision bf16x3|bf16|fp32] [--no-cpu-baseline]
+                  [--scaling weak|strong] [--precision bf16x3|bf16|fp32] [--no-cpu-baseline] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one synthetic batch.  Workloads (BASELINE.json `configs`, 0-based):
   c2 (default) configs[1]: pixel indices -> learnable-camera rays -> NDC -> stratified + importance sampling -> coarse +
@@ -322,6 +322,7 @@ class NerfWorkload:
         prd, _ = proj_ray_dist_loss_single(kps0_list=self.kps0, kps1_list=self.kps1, img_idx0=i, img_idx1=j, rays0=ri,
                                            rays1=rj, mode="train", device=self.kps0.device, H=H, W=W, args=self.args,
                                            camera_model=cam, method="NeRF", i_map=np.arange(synth.FERN_NCAM))
+        self.prd = prd.detach()
         (C["prd_weight"] * prd).backward()                 # accumulates into the flat buffer (assign_grads)
         eng.step_host(zero=False) if on_host else eng.step_device(zero=False)
         self.grads.all_reduce_mean()
@@ -404,10 +405,46 @@ def kernel_breakdown(lib, wl, steps, w, burst, sustained, hbm, src):
     return out, other / steps, tj
 
 
+def dump_outputs(wl, out_dir):
+    """Write what a caller of the timed step holds after its last call, one ``<name>.npy`` (float32) per array: the
+    loss (for c3 also ``loss.prd``, the PRD term), every parameter gradient after the all-reduce as
+    ``grad.<module>.<parameter>`` and, for c3, whose step ends in the optimiser, the updated parameters as
+    ``param.<module>.<parameter>``.  The inputs are seeded, so two builds run with the same arguments can be compared
+    array for array.  c2, c4 and c5 start every step from the same parameters, so round-off does not accumulate (c2 on
+    a B200: 4e-7 of each tensor's max after 20 steps); c3 feeds each step's round-off back
+    through the optimiser and the threshold-masked PRD loss, so its dumps drift apart step by step (on a B200, camera
+    parameters 2e-10 apart after the first step, 7e-4 after the seventh): compare c3 with few steps."""
+    m = wl.mods
+    if "nets" in m:
+        nets = {f"net{k}.{s}": getattr(net, s + "_net") for k, net in enumerate(m["nets"]) for s in ("fg", "bg")}
+    else:
+        nets = {"coarse": m["coarse"], "fine": m["fine"]}
+    out = {"loss": wl.eng.loss_dev}
+    if wl.wname == "c3":
+        out["loss.prd"] = wl.prd
+    for key, g in wl.grads.views.items():          # flat-buffer keys: "<module>.<field tensor index>", "camera.<name>"
+        prefix, _, i = key.rpartition(".")
+        if prefix == "camera":
+            name, p = key, getattr(m["cam"], i)
+        else:
+            p = nets[prefix].field_tensors()[int(i)]
+            name = prefix + "." + next(n for n, q in nets[prefix].named_parameters() if q is p)
+        out["grad." + name] = g
+        if wl.wname == "c3":
+            out["param." + name] = p
+    out = {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed steps; --impl reference stops early once 240 s of wall time are used (its JSON line "
+                         "reports the steps it timed as steps_timed)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -416,7 +453,12 @@ def main():
                     help="bf16x3 (default: split-bf16 tensor-core path, the parity-grade mode) | bf16 | fp32")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-inference", action="store_true", help="skip the forward-only section (ncu launch lists of the timed step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and gradients of the last one (and, for c3, the updated "
+                         "parameters) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 step (--impl b200)")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -460,6 +502,8 @@ def main():
     with ClockSampler(local) as clk:
         ms_dev = timed(False, args.steps)
     launches = int(lib.scnerf_launch_count(1))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
     for _ in range(2):
         wl.step(True)
     ms_e2e = timed(True, args.steps)
